@@ -14,6 +14,9 @@ spectrogram -> KL-NMF -> all-TDOA GCC-NMF argmax mask -> masked reconstruction -
 `--impl reference` times the reference's own CPU algorithm (the numpy oracle port: the reference is
 pure Python and /root/reference does not exist on the GPU box) on this box's host cores, on the same
 30 s clip per step, BLAS threads pinned and recorded, steps bounded by a time budget.
+
+`--dump-outputs DIR` writes what the last timed step returned (on rank 0) as DIR/<name>.npy, so that two builds can be
+compared output for output on the same seeded inputs.
 """
 import argparse
 import json
@@ -37,6 +40,7 @@ NMF_ITERATION_DRAM_BYTES = 39.7e6
 EXECUTED_PRODUCTS = 3.5
 METRIC = 'STFT frames/sec (1024-FFT, K=1024) full GCC-NMF pipeline'
 UNIT = 'frames/s'
+DUMP_LIMIT_BYTES = 64 * 1000 * 1000
 
 
 def workload_config(n_gpus):
@@ -186,6 +190,32 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------ GPU arm
+def host_outputs(r):
+    """The public entries of a step's result dict copied to the host: complex tensors as (..., 2) real / imaginary pairs in
+    their own precision, float64 kept, integers as float64 (exact), everything else float32.  Above DUMP_LIMIT_BYTES in all,
+    every array is reduced to the same fixed stride of its flattened elements."""
+    import torch
+    out = {}
+    for name, v in r.items():
+        if name.startswith('_'):
+            continue
+        t = torch.as_tensor(v).detach().cpu()
+        if t.is_complex():
+            t = torch.view_as_real(t)
+        dtype = torch.float64 if t.dtype == torch.float64 or not t.is_floating_point() else torch.float32
+        out[name] = t.to(dtype).contiguous().numpy()
+    stride = -(-sum(a.nbytes for a in out.values()) // DUMP_LIMIT_BYTES)
+    if stride > 1:
+        out = {name: np.ascontiguousarray(a.ravel()[::stride]) for name, a in out.items()}
+    return out
+
+
+def write_outputs(directory, outputs):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(directory, name + '.npy'), a)
+
+
 def load_peaks():
     p = os.path.join(ROOT, 'MEASURED_PEAKS.json')
     if os.path.exists(p):
@@ -273,6 +303,8 @@ def run_gpu(args):
     wall = time.perf_counter() - wall0
     windows.append((wall0, wall0 + wall))
     launches = h.launches - launches0
+    # copied now: the result dict holds views of buffers that the later (untimed) calls overwrite
+    outputs = host_outputs(r) if args.dump_outputs and rank == 0 else None
     total_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device=h.device)
     if world > 1:
         dist.all_reduce(total_ms, op=dist.ReduceOp.MAX)
@@ -346,6 +378,8 @@ def run_gpu(args):
         }
         if world == 1 and not args.no_cpu_baseline:
             line['cpu_baseline'] = cpu_baseline(20.0)      # 10-15 s of CPU work on the host cores (bounded sample of the same clip)
+        if outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -358,7 +392,13 @@ def main():
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs of the last timed step as DIR/<name>.npy (float32 / float64, at most 64 MB in all)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the b200 arm')
     if args.impl == 'reference':
         run_reference(args)
     else:
